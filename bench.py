@@ -20,6 +20,9 @@ packed (cost,d) minima -> final maps) is a fused reduce-scatter + all-gather ove
   cpu_baseline / --impl reference : the reference's pthreads CPU path on the host cores: oracle/_ref (the
              reference's own CVC/CVF/DispSel sources compiled against an OpenCV shim) when it was built,
              else the C port; a bounded slice sample per step, all cores and the reference's 8-thread cap
+
+--dump-outputs DIR writes what the timed path computed in its last step (both disparity maps, float32 .npy); the
+frame is generated from a fixed seed per workload, so two builds can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -213,7 +216,12 @@ def main():
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "p2p-barrier", "nccl"],
                     help="N>1: p2p = fused WTA + exchange over NVLink peer memory, ordered by device-side flags; "
                          "p2p-barrier = same kernels separated by NCCL barriers; nccl = local WTA then ncclAllGather")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the disparity maps of the last timed step as DIR/lDisMap.npy and "
+                         "DIR/rDisMap.npy (float32, H x W) on rank 0, to compare two builds on the same seeded frame")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.emulate_shards > 1):
+        ap.error("--dump-outputs needs the product path (--impl ours) without --emulate-shards")
     W, H, D = WORKLOADS[args.workload]
     WORKLOAD = workload_name(args.workload)
 
@@ -362,12 +370,34 @@ def main():
             out.append(de.stage_ms(4))
         return out
 
+    def dump_maps(out_dir):
+        """Both u8 disparity maps of the last step, read where that step left them (the context's device maps; with
+        the fused p2p exchange, the complete maps in the exchange block), saved as float32 .npy."""
+        if p2p is not None:
+            p2p.fetch(lmap.data_ptr(), rmap.data_ptr())
+            de.sync()
+            maps = [lmap.numpy().copy(), rmap.numpy().copy()]
+        else:
+            maps = []
+            for what in (2, 3):
+                ptr, pitch = C.c_void_p(), C.c_size_t()
+                capi.check(L.psm_device_ptr(de.handle, what, C.byref(ptr), C.byref(pitch)), de.handle)
+                view = type("DeviceMap", (), {"__cuda_array_interface__": {
+                    "shape": (H, W), "typestr": "|u1", "data": (ptr.value, False), "strides": (pitch.value, 1),
+                    "version": 2}})()
+                maps.append(torch.as_tensor(view, device="cuda").cpu().numpy())
+        os.makedirs(out_dir, exist_ok=True)
+        for name, m in zip(("lDisMap", "rDisMap"), maps):
+            np.save(os.path.join(out_dir, f"{name}.npy"), m.astype(np.float32))
+
     launches0 = de.launch_count()
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
     total_ms = timed(False, args.steps)
     launches_per_step = (de.launch_count() - launches0) // (warm + args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_maps(args.dump_outputs)
     kms = kernel_times(args.steps)
     clocks = sampler.stop() if rank == 0 else None
     stage = {n: de.stage_ms(i) for i, n in enumerate(["ingest", "cvc", "cvf", "wta", "cvf_kernel"])}

@@ -1,9 +1,12 @@
-"""CPU-only: the parts of bench.py that run without a GPU keep the driver's contract -- the reference arm prints one JSON
-line with the agreed keys (rank 0 only), and the product arm refuses to run without a CUDA device (no CPU fallback)."""
+"""CPU-only: the parts of bench.py that run without a GPU keep their interface -- the reference arm prints one JSON
+line with the agreed keys (rank 0 only), and the product arm refuses to run without a CUDA device (no CPU fallback).
+GPU: --dump-outputs writes the maps the timed path computed."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 from conftest import ROOT
 
@@ -35,6 +38,35 @@ def test_reference_arm_is_silent_on_other_ranks():
     p = run(["--impl", "reference", "--workload", "C3", "--steps", "1", "--warmup", "0", "--gpus", "2"],
             env={"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"})
     assert p.returncode == 0 and p.stdout.strip() == ""
+
+
+def test_dump_outputs_needs_the_product_path(tmp_path):
+    for extra in (["--impl", "reference"], ["--emulate-shards", "2"]):
+        p = run(["--steps", "1", "--warmup", "0", "--dump-outputs", str(tmp_path / "out")] + extra)
+        assert p.returncode != 0 and "--dump-outputs" in p.stderr
+    assert not (tmp_path / "out").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_maps_of_the_timed_path(tmp_path):
+    """--dump-outputs writes both disparity maps of the last timed step; they equal the maps the C-ABI gives
+    for the same seeded frame."""
+    import numpy as np
+    from primestereomatch_b200 import DispEst, synth
+    from bench import WORKLOADS
+    p = run(["--workload", "C3", "--steps", "2", "--warmup", "0", "--no-cpu-baseline", "--no-parity",
+             "--dump-outputs", str(tmp_path / "out")])
+    assert p.returncode == 0, p.stderr[-2000:]
+    W, H, D = WORKLOADS["C3"]
+    l, r, _ = synth.stereo_pair_f32(W, H, D)
+    with DispEst(l, r, D) as de:
+        de.CostConst_GPU(); de.CostFilter_GPU(); de.DispSelect_GPU()
+        want = {"lDisMap": de.lDisMap.copy(), "rDisMap": de.rDisMap.copy()}
+    assert sorted(os.listdir(tmp_path / "out")) == ["lDisMap.npy", "rDisMap.npy"]
+    for name, m in want.items():
+        got = np.load(tmp_path / "out" / f"{name}.npy")
+        assert got.dtype == np.float32 and got.shape == (H, W)
+        assert np.array_equal(got, m.astype(np.float32)), name
 
 
 def test_product_arm_needs_a_gpu():
